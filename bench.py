@@ -19,7 +19,12 @@ Weak scaling: every rank plans its own share, so `--gpus 8` runs c4 / c5 exactly
 
 After the timed regions (never inside them) rank 0 adds: `parity_check` (environments OF THE TIMED BATCH re-planned
 with explicit noise and compared with the CPU oracle), `cpu_baseline`, and `gpu_baseline` (the same algorithm as
-batched eager PyTorch / cuBLAS on this GPU, and the reference's own `_plan` on this GPU when baseline/_ref exists).
+batched eager PyTorch / cuBLAS on this GPU, and the reference's own `_plan` on this GPU when TDMPC2_REFERENCE_DIR names
+a reference checkout).
+
+--dump-outputs DIR writes what the last timed step returned to its caller: DIR/actions.npy, float32 [global envs,
+action_dim].  Inputs (weights, observations, noise seeds) depend only on the arguments, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -31,6 +36,7 @@ import subprocess
 import sys
 import tempfile
 import time
+from typing import Optional
 
 import torch
 
@@ -45,6 +51,7 @@ UNIT = "steps/s"
 WORKLOAD = "c2"
 SHARDS = {"c2": 1, "c3": 1, "c4": 8, "c5": 8}               # BASELINE.json: c4 / c5 are stated for 8 GPUs
 CPU_THREADS = int(os.environ.get("TDMPC2_CPU_THREADS", "8"))    # intra-op threads per reference process
+DUMP_BYTES = 64 << 20                                        # --dump-outputs: most bytes written in all
 
 
 def bench_cfg(name: str, envs=None):
@@ -59,6 +66,20 @@ def describe(name: str, cfg, E_local: int) -> str:
     model = {"c2": "dog-run 5M", "c3": "humanoid-walk 48M", "c4": "mt80 317M", "c5": "mt80 317M"}.get(name, name)
     return (f"{name}: {model} model, {E_local} envs/GPU, num_samples={cfg.num_samples}, horizon={cfg.horizon}, "
             f"iterations={cfg.iterations}")
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Each array as out_dir/<name>.npy in float32, DUMP_BYTES in all at most: an array over its share keeps a sample of
+    its rows drawn from a fixed seed, so runs with the same arguments store the same rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = a.detach().to("cpu", torch.float32)
+        if a.numel() * 4 > share:
+            rows = max(1, share // (4 * a[0].numel()))
+            a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def load_peaks():
@@ -146,7 +167,7 @@ def _cpu_worker(args):
         agent = ref_harness.build_agent(cfg, sd)
         th.manual_seed(3 + seed)
         for s in range(warmup + steps):
-            if times and time.perf_counter() - t_begin > budget_s:
+            if budget_s is not None and times and time.perf_counter() - t_begin > budget_s:
                 break
             t = time.perf_counter()
             for e in range(envs):
@@ -160,7 +181,7 @@ def _cpu_worker(args):
         model = OracleModel(cfg, sd)
         prev = th.zeros(envs, cfg.horizon, cfg.action_dim)
         for s in range(warmup + steps):
-            if times and time.perf_counter() - t_begin > budget_s:
+            if budget_s is not None and times and time.perf_counter() - t_begin > budget_s:
                 break
             noise = draw_noise(cfg, 3 + 1000 * s + seed, envs)
             t = time.perf_counter()
@@ -188,12 +209,14 @@ def _cpu_layout_run(wl, steps, warmup, budget_s, procs, threads, use_ref):
     return value, t_env, res[0][1]
 
 
-def cpu_reference_run(wl: str, steps: int, warmup: int, budget_s: float):
+def cpu_reference_run(wl: str, steps: int, warmup: int, budget_s: Optional[float]):
     """The reference's plan() on the host cores, with all the threads it can USE: eager PyTorch on these GEMM sizes
     stops scaling far below a 100+ core host (round 1: 128 threads in one process -> 53 s/plan, 16 -> 57 ms), and
     environments are independent, so the host layouts tried are processes x intra-op threads -- one process with
     16 threads, and process-parallel with 8 threads each over all cores -- and the BEST aggregate is reported.
     Every process plans its environments one after another (evaluate.py's loop; the reference has no env axis).
+    budget_s bounds the time of a layout (a process stops after the step that crosses it, and the layouts after the
+    first are skipped when they would exceed it); None times exactly `steps` steps after `warmup` in every layout.
     Returns (steps/s aggregate, seconds per env-plan of one process, cores used, kind, procs, all layouts tried)."""
     host = os.cpu_count() or 1
     use_ref = _ref_available()
@@ -202,7 +225,7 @@ def cpu_reference_run(wl: str, steps: int, warmup: int, budget_s: float):
         layouts += [(host // 32, 8), (host // 8, 8)]
     tried, best, t_first = [], None, None
     for procs, threads in layouts:
-        if t_first is not None and 12.0 * t_first * (warmup + 1) > 2.0 * budget_s and procs > 1:
+        if budget_s is not None and t_first is not None and 12.0 * t_first * (warmup + 1) > 2.0 * budget_s and procs > 1:
             tried.append({"procs": procs, "threads": threads, "skipped": "would exceed the time budget"})
             continue
         value, t_env, kind = _cpu_layout_run(wl, steps, warmup, budget_s, procs, threads, use_ref)
@@ -215,18 +238,15 @@ def cpu_reference_run(wl: str, steps: int, warmup: int, budget_s: float):
 
 def run_reference(args):
     """`--impl reference`: the reference's own CPU implementation of the path on the box's host cores, all the threads
-    it can use, on a bounded sample of the same workload.  Under torchrun only rank 0 runs."""
+    it can use, on a bounded sample of the same workload: every process plans one environment for exactly --warmup,
+    then --steps steps.  Under torchrun only rank 0 runs."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     wl = args.workload
     cfg = bench_cfg(wl)
-    per_env_gflop = flops_per_env(cfg, heads_used=cfg.num_q) / 1e9
-    budget = 150.0 if per_env_gflop < 200 else 240.0
-    heavy = per_env_gflop > 1000                 # 317M presets: one env-plan is tens of seconds of host time
-    steps = 1 if heavy else max(1, min(args.steps, 20))
-    value, t_env, cores, kind, procs, tried = cpu_reference_run(wl, steps, 0 if heavy else min(args.warmup, 1), budget_s=budget)
-    src = ("the reference's own unmodified TDMPC2._plan (baseline/_ref via oracle/ref_harness.py)" if kind == "reference"
+    value, t_env, cores, kind, procs, tried = cpu_reference_run(wl, args.steps, args.warmup, budget_s=None)
+    src = ("the reference's own unmodified TDMPC2._plan (TDMPC2_REFERENCE_DIR via oracle/ref_harness.py)" if kind == "reference"
            else "oracle port of the reference algorithm (reference sources not on this box)")
     sample = (f"{procs} processes x {cores // procs} threads, each planning 1 environment of the workload per step, "
               f"sequentially inside a process (the reference has no env axis); {src}")
@@ -356,12 +376,12 @@ def gpu_baselines(wl, cfg, dev, budget_s=40.0):
             ms = statistics.median(times)
             out["reference_plan_eager_gpu"] = {"value": rcfg.num_samples * rcfg.horizon / (ms * 1e-3), "unit": UNIT,
                                                "ms_per_env_plan": ms, "calls": len(times),
-                                               "impl": "the reference's own unmodified TDMPC2._plan (baseline/_ref), eager, "
+                                               "impl": "the reference's own unmodified TDMPC2._plan (TDMPC2_REFERENCE_DIR), eager, "
                                                        "one environment per call (it has no env axis), fp32"}
             del agent
             torch.cuda.empty_cache()
         else:
-            out["reference_plan_eager_gpu"] = {"unavailable": "baseline/_ref (copy of the reference's planning files) not on this box"}
+            out["reference_plan_eager_gpu"] = {"unavailable": "no reference checkout (TDMPC2_REFERENCE_DIR)"}
     except Exception as e:
         out["reference_plan_error"] = repr(e)[:300]
     return out
@@ -414,10 +434,16 @@ def main():
     ap.add_argument("--passes", type=int, default=3, choices=[1, 3],
                     help="3 = fp32-parity arithmetic (the headline); 1 = the DECLARED NON-PARITY fast mode (one fp16 MMA per "
                          "product): its own line, dtype f16, parity_check reports the elite-flip rate instead of gating")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the actions the last timed step returned to DIR/actions.npy (float32)")
     args = ap.parse_args()
-    args.warmup = max(args.warmup, 3)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the actions of this build's timed path; --impl reference has none to write")
         return run_reference(args)
+    args.warmup = max(args.warmup, 3)
 
     import torch.distributed as dist
     from tdmpc2_b200.tdmpc2 import TDMPC2
@@ -505,6 +531,8 @@ def main():
     launches = agent.planner.launches - launches0
     ms_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"actions": actions_host})
 
     # ---- dominant kernel: one CEM-iteration launch, timed alone with events on its stream
     from tdmpc2_b200.planner import draw_noise

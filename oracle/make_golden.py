@@ -1,8 +1,8 @@
 """Mint golden vectors from the REFERENCE's own planner -- TEST INFRASTRUCTURE ONLY.
 
-Run in the build container (needs /root/reference):
+Needs a reference checkout (see oracle/ref_harness.py):
 
-    python -m oracle.make_golden            # writes tests/golden/*.npz
+    TDMPC2_REFERENCE_DIR=<checkout>/tdmpc2 python -m oracle.make_golden     # writes tests/golden/*.npz
 
 For each workload it builds synthetic weights (tdmpc2_b200.synth, seed in the
 fixture), loads them into the reference WorldModel via oracle/ref_harness.py and
@@ -60,9 +60,31 @@ CASES = {
 }
 
 
+# name -> workload whose state-dict layout (keys, shapes) the reference's own WorldModel is recorded for
+MODEL_KEY_CASES = {"tiny_rgb_keys": "tiny-rgb"}
+
+
+def mint_model_keys(out_dir, name, wl):
+    """The keys and shapes of the reference model for `wl`, in this project's naming (the harness stores the Q ensemble
+    as `_Qs.p.<layer>/<param>`; written here as `_Qs.params.<layer>.<param>`).  build_agent() asserts that the synthetic
+    state dict has exactly these keys and load_state_dict() that it has these shapes."""
+    cfg = workload(wl)
+    agent = rh.build_agent(cfg, synth_state_dict(cfg, seed=2))
+    sd = {(("_Qs.params." + k[len("_Qs.p."):].replace("/", ".")) if k.startswith("_Qs.p.") else k): v
+          for k, v in agent.model.state_dict().items()}
+    keys = sorted(sd)
+    np.savez_compressed(os.path.join(out_dir, name + ".npz"), workload=wl, keys=np.array(keys),
+                        shapes=np.array([",".join(str(d) for d in sd[k].shape) for k in keys]),
+                        torch_version=torch.__version__)
+    print(f"{name}: {len(keys)} keys -> tests/golden/{name}.npz")
+
+
 def main(only=None):
     out_dir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
+    for name, wl in MODEL_KEY_CASES.items():
+        if not only or name in only:
+            mint_model_keys(out_dir, name, wl)
     for name, (wl, over, wseed, perturb, emb_scale, calls) in CASES.items():
         if only and name not in only:
             continue

@@ -1,8 +1,8 @@
 """Harness that executes the REFERENCE's own planner code on CPU -- TEST INFRASTRUCTURE ONLY.
 
-Works only where the reference checkout exists (default /root/reference, i.e. in
-the build container; never on the GPU box).  Nothing from the reference is
-copied: its modules are imported from where they lie.  The recipe is the one
+Works only where a reference checkout is available: TDMPC2_REFERENCE_DIR names its
+tdmpc2/ package directory (the one holding tdmpc2.py).  Nothing from the reference
+is copied: its modules are imported from where they lie.  The recipe is the one
 verified in SURVEY.md section 8(c) / Appendix A:
 
   1. import-only stubs for `tensordict` (not installable here) so that
@@ -29,32 +29,11 @@ from typing import Dict, Optional
 import torch
 import torch.nn as nn
 
-_ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-# Where the reference's modules lie: the read-only checkout in the build container, or -- on the GPU box, where
-# /root/reference does not exist -- the git-ignored verbatim copy `baseline/_ref/tdmpc2` that `make_ref_copy()` (run by
-# __graft_entry__.build()) places next to the repo so that the unmodified reference can be timed beside the kernels.
-_CANDIDATES = [os.environ.get("TDMPC2_REFERENCE_DIR", ""), "/root/reference/tdmpc2",
-               os.path.join(_ROOT, "baseline", "_ref", "tdmpc2")]
-REF_DIR = next((d for d in _CANDIDATES if d and os.path.isfile(os.path.join(d, "tdmpc2.py"))), _CANDIDATES[1])
-
-
-def make_ref_copy(src: str = "/root/reference/tdmpc2") -> bool:
-    """Copy the files of the reference's planning path (tdmpc2.py + common/*.py, unmodified) to baseline/_ref/tdmpc2
-    (git-ignored, travels to the GPU box with the snapshot).  No-op where the checkout does not exist."""
-    import shutil
-    if not os.path.isfile(os.path.join(src, "tdmpc2.py")):
-        return False
-    dst = os.path.join(_ROOT, "baseline", "_ref", "tdmpc2")
-    os.makedirs(os.path.join(dst, "common"), exist_ok=True)
-    shutil.copy2(os.path.join(src, "tdmpc2.py"), os.path.join(dst, "tdmpc2.py"))
-    for f in os.listdir(os.path.join(src, "common")):
-        if f.endswith(".py"):
-            shutil.copy2(os.path.join(src, "common", f), os.path.join(dst, "common", f))
-    return True
+REF_DIR = os.environ.get("TDMPC2_REFERENCE_DIR", "")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REF_DIR, "tdmpc2.py"))
+    return bool(REF_DIR) and os.path.isfile(os.path.join(REF_DIR, "tdmpc2.py"))
 
 
 _mods = None
@@ -65,7 +44,7 @@ def _import_reference():
     if _mods is not None:
         return _mods
     if not available():
-        raise RuntimeError(f"reference checkout not found at {REF_DIR}")
+        raise RuntimeError(f"reference checkout not found: set TDMPC2_REFERENCE_DIR (now {REF_DIR!r})")
     if "tensordict" not in sys.modules:
         td = types.ModuleType("tensordict"); td.from_modules = None; td.TensorDict = dict
         tdnn = types.ModuleType("tensordict.nn"); tdnn.TensorDictParams = None

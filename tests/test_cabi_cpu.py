@@ -99,18 +99,21 @@ def test_world_model_state_dict_layout():
             assert torch.equal(m2.state_dict()[k], want[k]), k
 
 
-def test_pixel_model_keys_are_the_references():
-    """cfg.obs == 'rgb': the container's encoder keys are what the reference's own layers.conv registers
-    (_encoder.rgb.{2,4,6,8}.{weight,bias}, layers.py:136-150).  Needs the reference checkout (build container only)."""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference checkout not present")
+def test_pixel_model_keys_are_the_references(golden_dir):
+    """cfg.obs == 'rgb': the container's keys and shapes are what the reference's own WorldModel registers, its encoder
+    keys what layers.conv registers (_encoder.rgb.{2,4,6,8}.{weight,bias}, layers.py:136-150).  The reference's layout
+    is stored in tests/golden/tiny_rgb_keys.npz (oracle/make_golden.py mints it from the reference model)."""
+    import numpy as np
     from tdmpc2_b200.config import workload
     from tdmpc2_b200.synth import synth_state_dict
-    cfg = workload("tiny-rgb")
+    f = np.load(os.path.join(golden_dir, "tiny_rgb_keys.npz"), allow_pickle=False)
+    ref = {str(k): tuple(int(d) for d in str(s).split(",") if d) for k, s in zip(f["keys"], f["shapes"])}
+    cfg = workload(str(f["workload"]))
     sd = synth_state_dict(cfg, seed=2)
-    agent = ref_harness.build_agent(cfg, sd)                 # asserts key-for-key equality with the reference model
-    ref_keys = {k for k in agent.model.state_dict() if k.startswith("_encoder.")}
+    ours = {k: tuple(v.shape) for k, v in sd.items()        # the copies build_agent() leaves out of the reference model
+            if not k.startswith(("_detach_Qs_params.", "_target_Qs_params.")) and "__" not in k}
+    assert ours == ref
+    ref_keys = {k for k in ref if k.startswith("_encoder.")}
     assert ref_keys == {k for k in sd if k.startswith("_encoder.")} == {
         f"_encoder.rgb.{i}.{n}" for i in (2, 4, 6, 8) for n in ("weight", "bias")}
     with pytest.raises(ValueError):                          # layers.conv flattens [num_channels, 4, 4]
@@ -187,3 +190,19 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["host_cores"] == os.cpu_count()
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["gpu_launches"] == 0
     assert "workload" in line["config"]
+
+
+def test_bench_reference_arm_times_exactly_the_steps_asked(monkeypatch, capsys):
+    """`--impl reference --steps K --warmup W` plans W + K steps in every process: no cap on K, no time budget."""
+    import argparse, importlib.util, json
+    import oracle.plan_oracle as po
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    calls, real = [], po.plan_oracle
+    monkeypatch.setattr(po, "plan_oracle", lambda *a, **k: calls.append(1) or real(*a, **k))
+    monkeypatch.setattr(bench, "_ref_available", lambda: False)
+    monkeypatch.setattr(os, "cpu_count", lambda: 8)          # one host layout: one process, in this interpreter
+    bench.run_reference(argparse.Namespace(workload="c2", steps=23, warmup=2, gpus=1))
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+    assert len(calls) == 25 and line["steps"] == 23 and line["warmup"] == 2
